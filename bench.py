@@ -2,9 +2,12 @@
 16 kHz, n_fft=512, hop=256) for the workload `configs[1]`: batch = 256 x 4 s synthetic clips per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--precision auto|fp32|f16x3_tc|f16_tc] [--no-extras]
+                  [--dump-outputs DIR]
   python bench.py --impl reference      # the CPU arm (oracle port of the reference path, all host threads)
 
 One "step" = one pass of the hot path (stft -> model -> decompress/mask -> istft) over one batch.
+--dump-outputs DIR writes what the last of the K timed steps returned as DIR/<name>.npy (float32); the inputs and weights
+are fixed by their seeds, so two builds run with the same arguments can be compared output for output.
 `value` is measured with the inputs resident in HBM; `e2e` goes through the public API with pinned HOST
 buffers, the H2D copy of the waveforms and the D2H copy of the result inside the timed region.
 Multi-GPU: one process per GPU (torchrun), clips sharded over ranks, no data-path collective (weak
@@ -20,6 +23,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -29,6 +33,21 @@ SR, N_FFT, HOP, WIN = 16000, 512, 256, 512
 CLIP_SECONDS = 4
 FLOP_PER_FRAME_STEP_SB = 257 * 3_638_784  # SURVEY 8d: sub-band stack, per clip per LSTM step
 FLOP_PER_FRAME_STEP_ALL = 942_774_784
+DUMP_BYTES = 63 * 10**6  # array bytes --dump-outputs writes at most: under 64 MB in all with the .npy headers
+
+
+def dump_outputs(out_dir: str, arrays: dict, rank: int = 0, world: int = 1) -> None:
+    """Writes each tensor of ``arrays`` as out_dir/<name>.npy in float32 (<name>_rank<r>.npy with several ranks).  Where
+    they exceed this rank's share of DUMP_BYTES, every array keeps the same fixed, seeded sample of its leading (clip)
+    dimension, in order, so that repeated runs write the same sample."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total, budget = sum(a.nbytes for a in arrays.values()), DUMP_BYTES // world
+    for name, a in arrays.items():
+        if total > budget and a.ndim:
+            keep = a.shape[0] * budget // total
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}_rank{rank}.npy" if world > 1 else f"{name}.npy"), a)
 
 
 def load_peaks():
@@ -186,7 +205,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the `precisions`, `latency_b1` and `train_dp` objects")
     ap.add_argument("--no-train", action="store_true", help="skip the `train_dp` object")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                                                          "(float32; above 64 MB, a fixed, seeded sample of the clips)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA implementation (--impl b200)")
     if args.model == "fullsubnet_train":
         import bench_train
         return bench_train.main(args)
@@ -280,14 +305,16 @@ def main():
             ms = float(t.item())
         return ms / steps, [s / steps for s in stage]
 
+    last = {}  # output of the latest step_resident(): --dump-outputs writes the one of the last timed step
+
     def step_resident():
         if args.model == "fullsubnet":
-            model.enhance(x_dev, N_FFT, HOP, WIN)
+            last["enhanced"] = model.enhance(x_dev, N_FFT, HOP, WIN)
         elif args.model == "improved_fullsubnet":
             with torch.no_grad():
-                model(x_dev)  # wav -> wav (improved_fullsubnet/model.py:541-591)
+                last["enhanced"] = model(x_dev)  # wav -> wav (improved_fullsubnet/model.py:541-591)
         else:
-            inf.enhance_batch(x_dev)
+            last["enhanced"] = inf.enhance_batch(x_dev)
 
     def step_e2e():
         if args.model == "improved_fullsubnet":
@@ -303,6 +330,8 @@ def main():
     ms_step, _ = timed(step_resident, args.steps, args.warmup)
     clocks = sampler.stop()
     launches = int(lib.fsn_last_launch_count())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, rank, world)
     # second pass with stage events on (separate from the headline timing)
     _, stage_ms = timed(step_resident, max(2, min(args.steps, 3)), 1, prof=True)
     ms_e2e, _ = timed(step_e2e, args.steps, 1)
@@ -430,7 +459,7 @@ def main():
         torch.cuda.empty_cache()
         import bench_train
         targs = argparse.Namespace(**vars(args))
-        targs.batch, targs.steps, targs.warmup = 64, max(2, min(args.steps, 5)), 3
+        targs.batch, targs.steps, targs.warmup, targs.dump_outputs = 64, max(2, min(args.steps, 5)), 3, None
         tl = bench_train.measure(targs, dist, dev, rank, world, local, cpu_leg=False)
         line["train_dp"] = {k: tl[k] for k in ("value", "unit", "ms_per_step", "n_gpus", "dtype", "gpu_launches")}
         line["train_dp"].update({"workload": tl["config"]["workload"], "parallelism": tl["config"]["parallelism"],

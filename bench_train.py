@@ -86,7 +86,7 @@ def main(args):
 def measure(args, dist, dev, rank, world, local, cpu_leg=True):
     """One measurement of the training step on an initialised process group (``dist`` = torch.distributed or None);
     returns the JSON line as a dict.  bench.py embeds it as `train_dp` next to the inference numbers."""
-    from bench import ClockSampler, load_peaks, pick_cpu_threads
+    from bench import ClockSampler, dump_outputs, load_peaks, pick_cpu_threads
     from fullsubnet_b200 import _lib
     from fullsubnet_b200.fullsubnet.model import Model
     from fullsubnet_b200.loss import mse_loss
@@ -136,8 +136,10 @@ def measure(args, dist, dev, rank, world, local, cpu_leg=True):
             ms = float(t.item())
         return ms / steps
 
+    last = {}
+
     def step_resident():
-        trainer.train_step(dev_noisy, dev_clean)
+        last["loss"] = trainer.train_step(dev_noisy, dev_clean)
 
     def step_e2e():
         loss = trainer.train_step(host_noisy, host_clean)  # H2D of both waveforms inside
@@ -148,6 +150,8 @@ def measure(args, dist, dev, rank, world, local, cpu_leg=True):
     sampler.start()
     ms_step = timed(step_resident, args.steps, args.warmup)
     clocks = sampler.stop()
+    if args.dump_outputs:  # the loss of the last timed step and the parameters its Adam update left
+        dump_outputs(args.dump_outputs, dict(last, **{"param." + k: p for k, p in model.named_parameters()}), rank, world)
     n0 = lib.fsn_total_launch_count()
     step_resident()
     torch.cuda.synchronize()
@@ -229,4 +233,5 @@ if __name__ == "__main__":
     ap.add_argument("--batch", type=int, default=64)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss and parameters after the last timed step")
     main(ap.parse_args())

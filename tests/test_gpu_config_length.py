@@ -33,15 +33,15 @@ def check_fp(y, fp):
 def test_fullsubnet_4s_clip_both_weight_sets(golden, dev, tag, gain, precision, crm_tol):
     from fullsubnet_b200.fullsubnet.model import Model
     from oracle import fullsubnet_oracle as O
-    g = golden("model_full_4s")
+    g = golden(f"model_full_4s_{tag}")
     y = O.make_noisy(1, 64000, seed=40, speechlike=True)
     check_fp(y, g["y_fp"])
     m = Model(**O.DEFAULT_MODEL_ARGS, precision=precision)
     m.load_state_dict(O.make_state_dict(seed=0, sb_fc_gain=gain), strict=True)
     m = m.to(dev).eval()
     wav, crm = m.enhance(y.to(dev), return_crm=True)
-    e_crm, e_l2 = rel_max(crm.cpu(), g[f"{tag}_crm"]), rel_l2(crm.cpu(), g[f"{tag}_crm"])
-    e_wav = float(np.abs(wav.cpu().numpy() - g[f"{tag}_wav"]).max())
+    e_crm, e_l2 = rel_max(crm.cpu(), g["crm"]), rel_l2(crm.cpu(), g["crm"])
+    e_wav = float(np.abs(wav.cpu().numpy() - g["wav"]).max())
     print(f"fullsubnet 4 s {tag} {m._resolve_precision()}: cRM max-rel {e_crm:.2e} rel-l2 {e_l2:.2e}, wav max-abs {e_wav:.2e}")
     assert e_crm < crm_tol and e_l2 < crm_tol and e_wav < WAV_TOL
 
@@ -50,15 +50,15 @@ def test_fullsubnet_4s_single_pass_f16_mask_gate(golden, dev):
     """The opt-in single-pass mode at T = 251: cRM gate on both weight sets, waveform gate on W-a."""
     from fullsubnet_b200.fullsubnet.model import Model
     from oracle import fullsubnet_oracle as O
-    g = golden("model_full_4s")
     y = O.make_noisy(1, 64000, seed=40, speechlike=True).to(dev)
     for tag, gain in (("wa", 1.0), ("wb", WB_GAIN)):
+        g = golden(f"model_full_4s_{tag}")
         m = Model(**O.DEFAULT_MODEL_ARGS, precision="f16_tc")
         m.load_state_dict(O.make_state_dict(seed=0, sb_fc_gain=gain), strict=True)
         wav, crm = m.to(dev).eval().enhance(y, return_crm=True)
-        assert rel_max(crm.cpu(), g[f"{tag}_crm"]) < CRM_TOL and rel_l2(crm.cpu(), g[f"{tag}_crm"]) < CRM_TOL
+        assert rel_max(crm.cpu(), g["crm"]) < CRM_TOL and rel_l2(crm.cpu(), g["crm"]) < CRM_TOL
         if tag == "wa":
-            assert np.abs(wav.cpu().numpy() - g["wa_wav"]).max() < WAV_TOL
+            assert np.abs(wav.cpu().numpy() - g["wav"]).max() < WAV_TOL
 
 
 @pytest.mark.parametrize("prec", ["fp32", "tf32_tc"])

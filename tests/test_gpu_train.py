@@ -233,7 +233,7 @@ def test_blocked_weight_gradient_gemm_matches_truncated_reference(dev):
         assert err < 1e-4, (M, N, K, a0, b0, err)
 
 
-def test_reference_trainer_flow_ddp_autocast_gradscaler(golden, dev):
+def test_reference_trainer_flow_ddp_autocast_gradscaler(golden, dev, tmp_path):
     """The reference's own optimisation flow (fullsubnet/trainer.py:56-69, base_trainer.py:32,46) on the drop-in Model:
     DistributedDataParallel (NCCL, world 1) + autocast + GradScaler + unscale_ + clip_grad_norm_ + torch.optim.Adam,
     two steps, equal to the golden steps of the unmodified reference."""
@@ -248,7 +248,9 @@ def test_reference_trainer_flow_ddp_autocast_gradscaler(golden, dev):
     args = small_args()
     core = build(args, O.make_state_dict(seed=7, args=args, sb_fc_gain=8.0), dev, "fp32")
     os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
-    os.environ.setdefault("MASTER_PORT", "29541")
+    if "MASTER_PORT" not in os.environ:  # a free port: other jobs on the host may hold any fixed one
+        import socket
+        s = socket.socket(); s.bind(("127.0.0.1", 0)); os.environ["MASTER_PORT"] = str(s.getsockname()[1]); s.close()
     created = not dist.is_initialized()
     if created:
         dist.init_process_group("nccl", rank=0, world_size=1, device_id=dev)
@@ -281,7 +283,7 @@ def test_reference_trainer_flow_ddp_autocast_gradscaler(golden, dev):
                 assert np.abs(v.cpu().numpy() - g[f"p{it}." + k]).max() < 2e-5, (it, k)
         # the Trainer accepts the DDP-wrapped model (no second all-reduce, checkpoints without the `module.` prefix)
         from fullsubnet_b200.trainer import Trainer
-        cfg = {"meta": {"use_amp": True, "save_dir": "/tmp/fsn_t", "experiment_name": "ddp"},
+        cfg = {"meta": {"use_amp": True, "save_dir": str(tmp_path), "experiment_name": "ddp"},
                "acoustics": {"n_fft": 64, "hop_length": 32, "win_length": 64},
                "trainer": {"train": {"epochs": 1, "save_checkpoint_interval": 1, "clip_grad_norm_value": 10}}}
         tr = Trainer(dist, 0, cfg, False, False, model, loss_function, optimizer, [(g["noisy"], g["clean"])], None)
@@ -289,7 +291,7 @@ def test_reference_trainer_flow_ddp_autocast_gradscaler(golden, dev):
         l3 = tr.train_step(torch.from_numpy(g["noisy"]), torch.from_numpy(g["clean"]))
         assert torch.isfinite(l3)
         tr._save_checkpoint(1)
-        ck = torch.load("/tmp/fsn_t/ddp/checkpoints/latest_model.tar", map_location="cpu")
+        ck = torch.load(tmp_path / "ddp" / "checkpoints" / "latest_model.tar", map_location="cpu")
         assert all(not k.startswith("module.") for k in ck["model"])
     finally:
         if created:

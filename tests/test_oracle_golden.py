@@ -246,10 +246,17 @@ def test_libcall_port_is_the_reference_computation(golden):
     from oracle import libcall_port as P
     g = golden("model_full")
     y = T(g["y"])
-    for tag, gain in (("wa", 1.0), ("wb", WB_GAIN)):
-        wav, crm = P.enhance(y, P.LibcallModel(O.make_state_dict(seed=0, sb_fc_gain=gain)), return_crm=True)
-        assert rel_max(crm, g[f"{tag}_crm"]) < 1e-6
-        assert np.abs(wav.numpy() - g[f"{tag}_wav"]).max() < 1e-6
+    # the fixtures were made on 8 threads (make_golden.py); the LSTM's CPU GEMMs split their sums by the thread count,
+    # so other counts move the waveform by a few 1e-6
+    threads = torch.get_num_threads()
+    torch.set_num_threads(8)
+    try:
+        for tag, gain in (("wa", 1.0), ("wb", WB_GAIN)):
+            wav, crm = P.enhance(y, P.LibcallModel(O.make_state_dict(seed=0, sb_fc_gain=gain)), return_crm=True)
+            assert rel_max(crm, g[f"{tag}_crm"]) < 1e-6
+            assert np.abs(wav.numpy() - g[f"{tag}_wav"]).max() < 1e-6
+    finally:
+        torch.set_num_threads(threads)
 
 
 def _fingerprint(y):
@@ -259,15 +266,15 @@ def _fingerprint(y):
 
 def test_oracle_at_config_length_4s(golden):
     """T = 251 (BASELINE configs 0/1 clip length), both weight sets: oracle vs the unmodified reference."""
-    g = golden("model_full_4s")
     y = O.make_noisy(1, 64000, seed=40, speechlike=True)
-    assert np.allclose(_fingerprint(y), g["y_fp"], rtol=0, atol=1e-9)
     torch.set_num_threads(8)
     for tag, gain in (("wa", 1.0), ("wb", WB_GAIN)):
+        g = golden(f"model_full_4s_{tag}")
+        assert np.allclose(_fingerprint(y), g["y_fp"], rtol=0, atol=1e-9)
         with torch.no_grad():
             wav, crm = O.enhance(y, O.make_state_dict(seed=0, sb_fc_gain=gain), return_crm=True)
-        assert rel_max(crm, g[f"{tag}_crm"]) < 5e-5 and rel_l2(crm, g[f"{tag}_crm"]) < 5e-5
-        assert np.abs(wav.numpy() - g[f"{tag}_wav"]).max() < 1e-4
+        assert rel_max(crm, g["crm"]) < 5e-5 and rel_l2(crm, g["crm"]) < 5e-5
+        assert np.abs(wav.numpy() - g["wav"]).max() < 1e-4
 
 
 def test_gru_oracle_matches_reference(golden):
